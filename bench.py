@@ -1,7 +1,7 @@
 """bench.py -- images/s of the YOLOv5 hot path on B200 (BASELINE.json metric: images/sec @640 at 1/2/4/8 GPUs + NMS us/img +
 conv tensor-pipe fraction).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config3|yolov5s|...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config3|yolov5s|...] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[2] ("config3", the configuration the >= 2x / >= 70 % targets are quoted on):
 yolov5l, 64 images of 640x640, bf16, forward + non_max_suppression through the public API of yolov5_b200.
@@ -260,11 +260,31 @@ def timed(D: Dist, fn, steps, sampler=None):
     return e0.elapsed_time(e1)
 
 
+DUMP_ELEMS = 2 << 20  # elements kept of a large output (8 MB of float32 + 16 MB of float64 positions)
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy (float32, or float64 for integer data).  Large tensors are reduced to
+    DUMP_ELEMS elements at seeded positions, stored beside them as <name>_index.npy, so two builds of the project can be
+    compared element for element on the same inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_ELEMS:
+            flat = t.reshape(-1)
+            pos = np.sort(np.random.RandomState(0).choice(flat.numel(), DUMP_ELEMS, replace=False))
+            t = flat[torch.from_numpy(pos).to(flat.device)]
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), pos.astype(np.float64))
+        t = t.cpu()
+        np.save(os.path.join(out_dir, f"{name}.npy"), (t.double() if not t.is_floating_point() else t.float()).numpy())
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # inference leg
 # ---------------------------------------------------------------------------------------------------------------------
-def infer_leg(D: Dist, model_name, bs, size, dt, steps, warmup, extras=True, cpu_base=True, sustain_s=0.0, tag=""):
-    """forward + NMS on `bs` images per rank.  Returns the record dict on rank 0 (None elsewhere)."""
+def infer_leg(D: Dist, model_name, bs, size, dt, steps, warmup, extras=True, cpu_base=True, sustain_s=0.0, tag="", dump_dir=None):
+    """forward + NMS on `bs` images per rank.  Returns the record dict on rank 0 (None elsewhere).  With `dump_dir`, rank 0
+    writes what the last timed step returned (see dump_outputs)."""
     from yolov5_b200 import _lib
     from yolov5_b200.cfg import model_cfg
     from yolov5_b200.models.yolo import DetectionModel, SegmentationModel
@@ -283,9 +303,12 @@ def infer_leg(D: Dist, model_name, bs, size, dt, steps, warmup, extras=True, cpu
     host_u8 = [torch.from_numpy(synth_images_u8(bs, size, 1000 + 10 * rank + i)).pin_memory() for i in range(n_rot)]
     dev_in = [(h.to(dev).to(TDT[dt]) / 255) for h in host_u8]
 
-    def step(i):
+    def step(i, keep=None):
         z = model(dev_in[i % n_rot])[0]
-        return nms_device(z, **nms_kw)  # device-side result (rows, idx, count): no host sync inside `value`
+        out = nms_device(z, **nms_kw)  # device-side result (rows, idx, count): no host sync inside `value`
+        if keep is not None:
+            keep.update(z=z, nms=out)
+        return out
 
     for i in range(warmup):
         out = step(i)
@@ -295,9 +318,15 @@ def infer_leg(D: Dist, model_name, bs, size, dt, steps, warmup, extras=True, cpu
     # ---------------- value: device-resident inputs ----------------
     sampler = ClockSampler(D.local) if rank == 0 else None
     l0 = _lib.launch_count()
-    ms_total = timed(D, step, steps, sampler)
+    last = {}
+    ms_total = timed(D, lambda i: step(i, last if i == steps - 1 else None), steps, sampler)
     clocks = sampler.stop() if sampler is not None else None
     eager_launches = _lib.launch_count() - l0
+    if dump_dir and rank == 0:  # the last timed batch: model(x)[0] and what non_max_suppression returns for it, images concatenated
+        rows, idx, cnt = last["nms"]
+        dump_outputs(dump_dir, {"predictions": last["z"], "detections_per_image": cnt,
+                                "detections": torch.cat([rows[b, :c] for b, c in enumerate(cnt.tolist())]),
+                                "detection_indices": torch.cat([idx[b, :c] for b, c in enumerate(cnt.tolist())])})
     prog = model._program(dev_in[0])
     graph_launches = len(prog.ops) * steps if prog.graph is not None else 0
     images, worst_ms = aggregate_throughput(bs * steps, ms_total, dev)
@@ -496,7 +525,7 @@ def torch_cuda_reference(cfg, sd, dev_in, dt, steps, dev):
 # ---------------------------------------------------------------------------------------------------------------------
 # training leg (BASELINE configs[3])
 # ---------------------------------------------------------------------------------------------------------------------
-def train_leg(D: Dist, model_name, bs, size, dt, steps, warmup, extras=True):
+def train_leg(D: Dist, model_name, bs, size, dt, steps, warmup, extras=True, dump_dir=None):
     """images/s of one optimisation step through the public API: model.train() under autocast, ComputeLoss, GradScaler-scaled
     backward, fused un-scale + clip + SGD-Nesterov (3 groups) + zero_grad (+ ModelEMA on rank 0, as train.py:251 does); per-GPU
     batch fixed, gradients averaged over ranks for N > 1 by FusedSGD.data_parallel -- one NCCL all-reduce of the packed arena -- with the
@@ -557,9 +586,19 @@ def train_leg(D: Dist, model_name, bs, size, dt, steps, warmup, extras=True):
         step(dev_img[i % n_rot], dev_tgt[i % n_rot])
     sampler = ClockSampler(D.local) if rank == 0 else None
     l0 = _lib.launch_count()
-    ms = timed(D, lambda i: step(dev_img[i % n_rot], dev_tgt[i % n_rot]), steps, sampler)
+    last = {}
+
+    def timed_step(i):
+        items = step(dev_img[i % n_rot], dev_tgt[i % n_rot])
+        if i == steps - 1:
+            last["items"] = items
+
+    ms = timed(D, timed_step, steps, sampler)
     clocks = sampler.stop() if sampler is not None else None
     launches = _lib.launch_count() - l0
+    if dump_dir and rank == 0:  # the last timed step's loss items and the parameters it left
+        dump_outputs(dump_dir, {"loss_items": last["items"],
+                                "parameters": torch.cat([q.detach().float().reshape(-1) for q in model.parameters()])})
     images, worst_ms = aggregate_throughput(bs * steps, ms, dev)
     value = images / (worst_ms / 1e3)
 
@@ -743,7 +782,12 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="override the per-GPU batch")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-subrecords", action="store_true", help="main workload only (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the main workload's outputs of its last timed step to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs records the outputs of --impl ours")
     a.warmup = max(a.warmup, 3)
     global _OUT
     _OUT = StdoutGuard()
@@ -789,11 +833,11 @@ def main():
     D.init()
     subs = not a.no_subrecords and a.workload == "config3"
     if train:
-        rec = train_leg(D, model_name, bs, size, dt, a.steps, a.warmup)
+        rec = train_leg(D, model_name, bs, size, dt, a.steps, a.warmup, dump_dir=a.dump_outputs)
         metric = "images/sec @640 (training step: forward + loss + backward + optimizer)"
     else:
         rec = infer_leg(D, model_name, bs, size, dt, a.steps, a.warmup, extras=True, cpu_base=not a.no_cpu_baseline,
-                        sustain_s=2.5 if subs else 0.0)
+                        sustain_s=2.5 if subs else 0.0, dump_dir=a.dump_outputs)
         metric = "images/sec @640 (forward + NMS)"
     sub = {}
     if subs:

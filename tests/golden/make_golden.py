@@ -517,9 +517,28 @@ def gen_ckpt():
           f"{os.path.getsize(f'{HERE}/ref_tiny.pt') / 1e6:.2f} MB")
 
 
+def gen_signatures():
+    """The reference's call signatures on the drop-in surface (parameter name, repr of the default, kind), which
+    tests/test_compat_cpu.py holds this package's callables against."""
+    import importlib
+    import inspect
+
+    from make_golden_cases import SIGNATURE_SURFACE
+
+    out = {}
+    for mod, qual in SIGNATURE_SURFACE:
+        obj = importlib.import_module(mod)
+        assert obj.__file__.startswith(REF), obj.__file__
+        for part in qual.split("."):
+            obj = getattr(obj, part)
+        out[f"{mod}:{qual}"] = [(n, repr(p.default) if p.default is not inspect.Parameter.empty else None, str(p.kind))
+                                for n, p in inspect.signature(obj).parameters.items()]
+    json.dump(out, open(f"{HERE}/ref_signatures.json", "w"), indent=1)
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["cfg", "model", "nms", "loss", "train", "post", "pre", "optim", "ckpt"]
+    which = sys.argv[1:] or ["cfg", "model", "nms", "loss", "train", "post", "pre", "optim", "ckpt", "signatures"]
     for w in which:
         {"cfg": gen_cfg, "model": gen_model, "nms": gen_nms, "loss": gen_loss, "train": gen_train, "post": gen_post, "pre": gen_pre,
-         "optim": gen_optim, "ckpt": gen_ckpt}[w]()
+         "optim": gen_optim, "ckpt": gen_ckpt, "signatures": gen_signatures}[w]()
     print("golden fixtures written to", HERE)

@@ -195,8 +195,6 @@ def test_bench_shape_config3_yolov5l_bs64_bf16(cuda):
     _check_model_batch_subset("yolov5l", 64, 640, torch.bfloat16, cuda, 31, 131)
 
 
-@pytest.mark.skipif(not os.environ.get("Y5_TEST_SHARDS"), reason="opt-in (Y5_TEST_SHARDS=1): written after the round's GPU budget was spent, "
-                    "never run on hardware yet")
 @pytest.mark.parametrize("batch", [32, 16, 8])
 def test_bench_shape_config3_shards(cuda, batch):
     """The per-GPU shards of config 3 when bench.py runs on 2 / 4 / 8 GPUs (64 images split over the ranks): other M extents,
